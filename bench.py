@@ -1,18 +1,17 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200 rasterizer (BASELINE.json: Mpix/s fwd+bwd @ 1M splats, 1600x1200).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C2] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step is one pass of the hot path over one synthetic camera: `_C.rasterize_gaussians` followed by
 `_C.rasterize_gaussians_backward` with fixed upstream gradients (SURVEY.md 8d).  Prints ONE JSON line (rank 0).
 
-Protocol (SURVEY.md 8d: median of >= 20 timed iterations after >= 5 warm-ups):
-  * a *window* is EXACTLY `--steps` iterations bracketed by barrier + torch.cuda.synchronize() on both sides, with a CUDA
-    event between consecutive iterations (on the launching stream); per iteration the time is the MAX over ranks;
-  * windows are repeated until at least `--min-time` seconds (default 0.5) and at least 20 iterations have been timed;
-  * `ms_per_step` = MEDIAN of all per-iteration times, `value` = W*H / that; min / median / max and the per-window means
-    are in `timing` so a perturbed window is visible instead of being averaged in;
+Protocol (SURVEY.md 8d: median of >= 20 timed iterations after >= 5 warm-ups; the defaults):
+  * each measured quantity is timed over EXACTLY `--steps` iterations, bracketed by barrier + torch.cuda.synchronize() on both
+    sides, with a CUDA event between consecutive iterations (on the launching stream); per iteration the time is the MAX over ranks;
+  * `ms_per_step` = MEDIAN of the per-iteration times, `value` = W*H / that; min / median / max are in `timing` so a perturbed
+    iteration is visible instead of being averaged in;
   * SM clocks / throttle reasons are sampled by a separate PROCESS (NVML, no GIL contention with the timed loop) that
     runs during every timed phase of the run.
   value        inputs resident in HBM
@@ -30,6 +29,8 @@ this path (BASELINE.md section 2), so its arm runs where it can -- on the GPU (s
 never imports the product's extension modules.
 N > 1: tile rows of the one image are sharded over the ranks (strong scaling); the screen-space gradient rows are
 exchanged once per backward.
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step of the resident path returned to its caller
+(see dump_outputs); the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -239,6 +240,35 @@ def algorithmic_bytes(P, Pv, R, N, T, M, coord, depth):
     }
 
 
+DUMP_PIXELS, DUMP_ROWS = 1 << 18, 1 << 16   # 15 image channels and 72 floats per Gaussian row: about 37 MB with the indices
+
+
+def dump_outputs(out_dir, fwd, grads, H, W, P):
+    """Write what one step of the resident path returned to its caller as out_dir/<name>.npy (float32; float64 for counts and
+    indices): the image maps (`color`, `alpha`, `depth`, ... as [C, pixels]), `radii` and `grad_<name>` for each gradient tensor.
+    Larger outputs are sampled: the same seeded DUMP_PIXELS pixels and DUMP_ROWS Gaussian rows every run, whose flat indices
+    are written as `pixel_index` and `row_index`.  The private state buffers are left out: their layout is the build's own."""
+    import numpy as np
+
+    def pick(n, k, seed):
+        return np.arange(n) if n <= k else np.sort(np.random.default_rng(seed).choice(n, size=k, replace=False))
+
+    pix, rows = pick(H * W, DUMP_PIXELS, 1), pick(P, DUMP_ROWS, 2)
+    out = {"num_rendered": np.array(int(fwd["num_rendered"]), np.float64), "pixel_index": pix.astype(np.float64), "row_index": rows.astype(np.float64)}
+    for k in ("color", "coord", "mcoord", "alpha", "normal", "depth", "mdepth"):
+        if k in fwd:
+            t = fwd[k]
+            out[k] = t.reshape(t.shape[0], -1)[:, torch.from_numpy(pix).to(t.device)].float().cpu().numpy()
+    per_row = {"radii": fwd["radii"]} if "radii" in fwd else {}
+    per_row.update({"grad_" + k: v for k, v in grads.items()})
+    for k, t in per_row.items():
+        out[k] = (t[torch.from_numpy(rows).to(t.device)] if t.shape[0] == P else t).float().cpu().numpy()
+    assert sum(v.nbytes for v in out.values()) <= 64 << 20
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -246,8 +276,8 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="C2")
-    ap.add_argument("--min-time", type=float, default=0.5, help="seconds of timed work per measured quantity (windows of --steps are repeated)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     a = ap.parse_args()
     a.warmup = max(a.warmup, 3)
     a.steps = max(a.steps, 1)
@@ -301,7 +331,7 @@ def main():
                                        out[10], out[11], out[4], coord, depth, False, slab[0], slab[1], True, H)
         g = C.rasterize_gaussians_backward_preprocess(acc, sc.bg, sc.means3D, out[8], E, sc.opacities, sc.scales, sc.rotations, 1.0, E, sc.viewmatrix,
                                                       sc.projmatrix, sc.tanfovx, sc.tanfovy, 0.0, H, W, sc.shs, 3, sc.campos, out[9], coord, depth, False)
-        return {"num_rendered": out[0]}, g
+        return {"num_rendered": out[0]}, dict(zip(rawapi.BWD_KEYS, g))
 
     def barrier():
         if multi:
@@ -309,31 +339,23 @@ def main():
         torch.cuda.synchronize()
 
     def measure(fn):
-        """Windows of exactly --steps iterations (barrier + synchronize on both sides, CUDA events between iterations on the
-        launching stream, max over ranks per iteration) until --min-time seconds and >= 20 iterations are on record."""
-        iters, windows, last, total = [], [], None, 0.0
+        """Exactly --steps iterations (barrier + synchronize on both sides, CUDA events between iterations on the launching
+        stream, max over ranks per iteration); returns their statistics and what the last one returned."""
         fn()                      # one more untimed step: the first call after a phase change pays one-off allocator / event set-up
         torch.cuda.synchronize()
-        while True:
-            ev = [torch.cuda.Event(enable_timing=True) for _ in range(a.steps + 1)]
-            barrier()
-            ev[0].record()
-            for i in range(a.steps):
-                last = fn()
-                ev[i + 1].record()
-            barrier()
-            t = torch.tensor([ev[i].elapsed_time(ev[i + 1]) for i in range(a.steps)] + [ev[0].elapsed_time(ev[a.steps])], device=dev, dtype=torch.float64)
-            if multi:
-                dist.all_reduce(t, op=dist.ReduceOp.MAX)
-            t = t.tolist()
-            iters += t[:-1]
-            windows.append(t[-1] / a.steps)
-            total += t[-1] * 1e-3
-            if (total >= a.min_time and len(iters) >= 20) or len(windows) >= 200:
-                break
-        med = statistics.median(iters)
-        return {"ms": med, "min_ms": min(iters), "max_ms": max(iters), "iterations": len(iters), "windows": len(windows),
-                "window_mean_ms": {"min": min(windows), "median": statistics.median(windows), "max": max(windows)}, "timed_s": total}, last
+        ev = [torch.cuda.Event(enable_timing=True) for _ in range(a.steps + 1)]
+        barrier()
+        ev[0].record()
+        for i in range(a.steps):
+            last = fn()
+            ev[i + 1].record()
+        barrier()
+        t = torch.tensor([ev[i].elapsed_time(ev[i + 1]) for i in range(a.steps)] + [ev[0].elapsed_time(ev[a.steps])], device=dev, dtype=torch.float64)
+        if multi:
+            dist.all_reduce(t, op=dist.ReduceOp.MAX)
+        t = t.tolist()
+        iters = t[:-1]
+        return {"ms": statistics.median(iters), "min_ms": min(iters), "max_ms": max(iters), "iterations": len(iters), "timed_s": t[-1] * 1e-3}, last
 
     import contextlib
     with (ClockSampler(local) if rank == 0 else contextlib.nullcontext()) as clk:
@@ -346,6 +368,9 @@ def main():
         ms_per_step = t_res["ms"]
         value = W * H / (ms_per_step * 1e-3) / 1e6
         R = int(last[0]["num_rendered"])
+        if a.dump_outputs and rank == 0:
+            dump_outputs(a.dump_outputs, *last, H, W, P)
+        del last
 
         # ---- end-to-end number: public autograd API, host inputs copied in, loss copied out ----
         # Host inputs of one training step, as train.py has them: the camera (matrices, position, background) and the
@@ -354,7 +379,8 @@ def main():
         r0, r1 = min(slab[0] * 16, H), min(slab[1] * 16, H)
         # multi-GPU: a rank's loss needs the ground-truth rows of its own slab only, so that is what it copies in
         host = {"view": sc_cpu.viewmatrix.pin_memory(), "proj": sc_cpu.projmatrix.pin_memory(), "campos": sc_cpu.campos.pin_memory(),
-                "bg": sc_cpu.bg.pin_memory(), "gt_color": (torch.rand(3, H, W) * 255).to(torch.uint8)[:, r0:r1].contiguous().pin_memory()}
+                "bg": sc_cpu.bg.pin_memory(),
+                "gt_color": (torch.rand(3, H, W, generator=torch.Generator().manual_seed(5678)) * 255).to(torch.uint8)[:, r0:r1].contiguous().pin_memory()}
         h2d = sum(v.numel() * v.element_size() for v in host.values())
         dbuf = {k: torch.empty_like(v, device=dev) for k, v in host.items()}
         leaves = {k: getattr(sc, k).clone().requires_grad_(True) for k in ("means3D", "scales", "rotations", "opacities", "shs")}
@@ -405,7 +431,7 @@ def main():
     roofline = roofline_issue = stages = step_hbm = None
     if ours and hasattr(C, "stage_timing"):
         C.stage_timing(True)
-        for _ in range(max(a.steps, 20)):
+        for _ in range(a.steps):
             step_resident()
         torch.cuda.synchronize()
         stages = C.stage_times()          # {name: (total_ms, launches)}
@@ -467,7 +493,7 @@ def main():
                        "parallelism": (f"tile-row slabs x{world}, gradient-row exchange: {exchange.mode}" + (f" over {exchange.window}" if exchange.window else "") + (f" (peer self-check failed: {exchange.fallback_reason})" if exchange.fallback_reason else "")
                                        if multi else "single GPU"),
                        "l2": "per-step working set (192 MB SH + 248 MB SH grads + 64 MB records + sort buffers) exceeds the 126 MB L2; no explicit flush",
-                       "protocol": f"median of {t_res['iterations']} per-iteration CUDA-event times ({t_res['windows']} windows of {a.steps} steps, barrier+synchronize around each window, max over ranks per iteration)"},
+                       "protocol": f"median of {t_res['iterations']} per-iteration CUDA-event times (one window of {a.steps} steps, barrier+synchronize around it, max over ranks per iteration)"},
             "timing": t_res,
             "e2e": {"value": e2e_value, "unit": "Mpix/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": 4, "ms_per_step": t_e2e["ms"], "timing": t_e2e,
                     "api": "GaussianRasterizer autograd module (what render() calls) + L1 vs 8-bit GT image + depth/normal/alpha regularisers; camera + GT image H2D from pinned memory every step (GT on a side stream), loss.item() D2H"},

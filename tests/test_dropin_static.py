@@ -1,41 +1,30 @@
 """Static drop-in check against the reference's own caller, `gaussian_renderer.render()` (reference
 gaussian_renderer/__init__.py:19-95): every name it imports from `diff_gaussian_rasterization`, every keyword it passes to
 `GaussianRasterizationSettings(...)` and to `rasterizer(...)`, and the 8-tuple it unpacks must exist in this repo's package.
-Runs on CPU where /root/reference is mounted; skipped elsewhere (the GPU box does not have the reference)."""
-import ast
+The call sites are recorded in tests/golden/render_call_sites.json (tools/gen_golden_render_calls.py)."""
 import inspect
+import json
 import os
 
-import pytest
-
-REF = "/root/reference/gaussian_renderer/__init__.py"
+from conftest import GOLDEN_DIR
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference checkout not present")
 def test_render_call_sites_fit_our_package():
     import diff_gaussian_rasterization as dgr
-    tree = ast.parse(open(REF).read())
-    imported = [a.name for n in ast.walk(tree) if isinstance(n, ast.ImportFrom) and n.module == "diff_gaussian_rasterization" for a in n.names]
+    with open(os.path.join(GOLDEN_DIR, "render_call_sites.json")) as f:
+        sites = json.load(f)
+    imported = sites["imports"]
     assert imported and all(hasattr(dgr, name) for name in imported), imported
     fields = set(dgr.GaussianRasterizationSettings._fields)
     fwd_params = set(inspect.signature(dgr.GaussianRasterizer.forward).parameters) - {"self"}
     integ_params = set(inspect.signature(dgr.GaussianRasterizer.integrate).parameters) - {"self"}
-    seen_settings = seen_call = 0
-    for node in ast.walk(tree):
-        if isinstance(node, ast.Call) and isinstance(node.func, ast.Name) and node.func.id == "GaussianRasterizationSettings":
-            kws = {k.arg for k in node.keywords}
-            assert kws <= fields, kws - fields
-            assert fields - kws == set() or kws, "render() must be able to build the settings tuple"
-            seen_settings += 1
-        if isinstance(node, ast.Call) and isinstance(node.func, ast.Name) and node.func.id == "rasterizer":
-            kws = {k.arg for k in node.keywords}
-            assert kws <= fwd_params, kws - fwd_params
-            seen_call += 1
-        if isinstance(node, ast.Call) and isinstance(node.func, ast.Attribute) and node.func.attr == "integrate":
-            kws = {k.arg for k in node.keywords}
-            assert kws <= integ_params, kws - integ_params
-    assert seen_settings >= 1 and seen_call >= 1
+    for kws in map(set, sites["settings_calls"]):
+        assert kws <= fields, kws - fields
+        assert fields - kws == set() or kws, "render() must be able to build the settings tuple"
+    for kws in map(set, sites["rasterizer_calls"]):
+        assert kws <= fwd_params, kws - fwd_params
+    for kws in map(set, sites["integrate_calls"]):
+        assert kws <= integ_params, kws - integ_params
+    assert len(sites["settings_calls"]) >= 1 and len(sites["rasterizer_calls"]) >= 1
     # render() unpacks 8 outputs from the rasterizer call (reference :71)
-    unpack = [n for n in ast.walk(tree) if isinstance(n, ast.Assign) and isinstance(n.targets[0], ast.Tuple) and isinstance(n.value, ast.Call)
-              and isinstance(n.value.func, ast.Name) and n.value.func.id == "rasterizer"]
-    assert unpack and len(unpack[0].targets[0].elts) == 8
+    assert sites["rasterizer_unpack"] and sites["rasterizer_unpack"][0] == 8

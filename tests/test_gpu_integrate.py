@@ -1,5 +1,5 @@
 """`GaussianRasterizer.integrate` (SURVEY.md 8f row 3) on the GPU against (1) the fixtures produced by the unmodified reference
-build, (2) the CPU oracle on fresh scenes, (3) the reference build itself on the box when present.
+build, (2) the CPU oracle on fresh scenes, (3) what the reference build computed on a larger load (hashed or sampled).
 
 Tolerances as in tests/test_oracle_integrate.py: integers, radii, projected coordinates and the points-per-pixel channel
 exact; float results 1e-4 (+1e-4 relative) with at most 1e-3 of the elements across an alpha threshold."""
@@ -13,6 +13,7 @@ import torch
 from conftest import INTEGRATE_CASES, ROOT, integrate_oracle_inputs, load_golden
 from test_oracle_integrate import close_with_outliers
 
+sys.path.insert(0, os.path.join(ROOT, "tools"))
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
 NAMES = ("color", "alpha_integrated", "color_integrated", "point_coordinate", "point_sdf", "radii")
@@ -116,15 +117,30 @@ def test_integrate_many_points_in_one_pixel_and_empty_inputs():
     assert (o[1] == 1.0).all() and (o[4] == -1000.0).all() and not o[2].any() and not o[0].any()
 
 
+def reference_build_scene():
+    """Mesh-extraction-like load: 50k splats, 9 points per splat (CPU tensors)."""
+    from gen_golden_refbuild import one_thread
+    with one_thread():
+        return _fresh_scene(50_000, 400, 304, 330.0, -3.0, 9, 450_000)
+
+
 def test_integrate_next_to_the_reference_build():
-    """Mesh-extraction-like load (50k splats, 9 points per splat) next to the reference's own kernel on the same GPU."""
-    import build_ref
-    if not os.path.exists(build_ref.target()):
-        pytest.skip("reference build oracle/_ref/ref_dgr_C.so not present on this box")
-    ref = build_ref.load()
-    sys.path.insert(0, os.path.join(ROOT, "tools"))
-    from gen_golden_integrate import call_reference
-    sc, pts = _fresh_scene(50_000, 400, 304, 330.0, -3.0, 9, 450_000)
+    """The mesh-extraction-like load against what the reference's own kernel computed on it (tests/golden/refbuild/integrate_50k.npz):
+    arrays compared bit for bit through their SHA-256, the others on a fixed sample of pixels and points."""
+    from gen_golden_refbuild import digest, scene_digest
+    sc, pts = reference_build_scene()
+    d = load_golden("refbuild/integrate_50k")
+    assert scene_digest(sc, pts) == str(d["inputs_sha256"]), "the scene recipe no longer makes the fixture's inputs"
     ours = _run_ours(sc, pts)
-    r = call_reference(ref, sc.to(DEV), pts.to(DEV), 3)
-    _check(ours, {k: v.cpu().numpy() for k, v in zip(NAMES, r[1:7])}, "ref-50k")
+    assert digest(ours["radii"]) == str(d["sha256_radii"])
+    assert digest(ours["point_coordinate"]) == str(d["sha256_point_coordinate"])
+    assert digest(ours["color"][8]) == str(d["sha256_points_per_pixel"])
+    assert not ours["color"][5].any()
+    color = ours["color"].reshape(9, -1)[:, d["pix"]]
+    for ch in (0, 1, 2, 3, 4, 6, 7):
+        close_with_outliers(color[ch], d["color"][ch], f"ref-50k/color[{ch}]")
+    for k in ("alpha_integrated", "color_integrated", "point_sdf"):
+        close_with_outliers(ours[k][d["pts"]], d[k], f"ref-50k/{k}")
+    untouched = ours["point_sdf"] == -1000.0
+    assert digest(untouched) == str(d["sha256_untouched"])
+    assert (ours["alpha_integrated"][untouched] == 1.0).all()
