@@ -5,7 +5,6 @@
 // 254-425, 429-571, 176-188; cuda_rasterizer/rasterizer_impl.h:22-94).
 #include <atomic>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
 #include <string>
@@ -70,31 +69,27 @@ static int debug_sync(const rgs_camera* cam, cudaStream_t s, const char* stage) 
 	return RGS_OK;
 }
 
-static GeomView carve_geom(char* base, int P, bool coord, size_t scan_bytes, size_t* total) {
+static GeomView carve_geom(char* base, int P, bool coord, size_t* total) {
 	Carver c(base);
 	GeomView g;
 	g.records = c.take<float>((size_t)P * rec_floats(coord));
 	g.depths = c.take<float>(P);
 	g.tiles_touched = c.take<uint32_t>(P);
-	g.offsets = c.take<uint32_t>(P);
+	g.bwd_rows = c.take<uint32_t>(P);
 	g.clamped = c.take<uint8_t>(P);
 	g.sigma_inv = c.take<float>((size_t)P * SIGMA_INV_FLOATS);
-	g.scan_temp = c.take<char>(scan_bytes);
-	g.scan_temp_bytes = scan_bytes;
+	g.bwd_row_count = c.take<uint32_t>(1);
 	if (total) *total = c.size();
 	return g;
 }
 
-static BinView carve_bin(char* base, size_t R, int tiles, size_t sort_bytes, size_t* total) {
+static BinView carve_bin(char* base, size_t R, int tiles, size_t* total) {
 	Carver c(base);
 	BinView b;
 	b.point_list = c.take<uint32_t>(R);
 	b.keys_sorted = c.take<uint64_t>(R);
 	b.hitmask = c.take<uint32_t>(hitmask_words(R, tiles));
-	b.point_list_unsorted = c.take<uint32_t>(R);
 	b.keys_unsorted = c.take<uint64_t>(R);
-	b.sort_temp = c.take<char>(sort_bytes);
-	b.sort_temp_bytes = sort_bytes;
 	if (total) *total = c.size();
 	return b;
 }
@@ -114,6 +109,14 @@ static ImgView carve_img(char* base, int grid_x, int grid_y, size_t N, bool coor
 	v.tile_diff = c.take<int>((size_t)(grid_x + 1) * (grid_y + 1));
 	if (total) *total = c.size();
 	return v;
+}
+
+// Height of the [C,Hs,W] maps one call stores: the whole image, or with compact_slab only the pixel rows of tile rows
+// [row_begin, row_end).
+static int stored_height(const rgs_camera* cam, int row_begin, int row_end) {
+	if (!cam->compact_slab) return cam->height;
+	const int hs = (row_end * TILE_Y < cam->height ? row_end * TILE_Y : cam->height) - row_begin * TILE_Y;
+	return hs > 0 ? hs : 0;
 }
 
 static int make_params(const rgs_camera* cam, const rgs_gaussians* g, FwdParams& p) {
@@ -142,13 +145,8 @@ static int make_params(const rgs_camera* cam, const rgs_gaussians* g, FwdParams&
 	p.row_begin = cam->tile_row_begin;
 	p.row_end = cam->tile_row_end < 0 ? p.grid_y : cam->tile_row_end;
 	if (p.row_begin < 0 || p.row_end > p.grid_y || p.row_begin > p.row_end) return fail(RGS_E_INVALID, "tile row slab out of range");
-	p.py_off = 0;
-	p.Hs = cam->height;
-	if (cam->compact_slab) {
-		p.py_off = p.row_begin * TILE_Y;
-		p.Hs = (p.row_end * TILE_Y < cam->height ? p.row_end * TILE_Y : cam->height) - p.py_off;
-		if (p.Hs < 0) p.Hs = 0;
-	}
+	p.py_off = cam->compact_slab ? p.row_begin * TILE_Y : 0;
+	p.Hs = stored_height(cam, p.row_begin, p.row_end);
 	p.tan_fovx = cam->tan_fovx;
 	p.tan_fovy = cam->tan_fovy;
 	// focal lengths computed on the host in float, as the reference does (rasterizer_impl.cu:288-289)
@@ -221,12 +219,11 @@ static int64_t forward_to_binning(const rgs_camera* cam, const FwdParams& p, int
 	if (!img_ptr) return fail(RGS_E_ALLOC, "image buffer callback returned NULL");
 	img = carve_img(img_ptr, p.grid_x, p.grid_y, N, p.coord, p.depth, nullptr);
 
-	const size_t scan_bytes = P > 0 ? scan_temp_bytes(P) : 0;
 	size_t geom_bytes = 0;
-	carve_geom(nullptr, P, p.coord, scan_bytes, &geom_bytes);
+	carve_geom(nullptr, P, p.coord, &geom_bytes);
 	char* geom_ptr = bufs->geom(bufs->geom_user, geom_bytes);
 	if (!geom_ptr) return fail(RGS_E_ALLOC, "geometry buffer callback returned NULL");
-	g = carve_geom(geom_ptr, P, p.coord, scan_bytes, nullptr);
+	g = carve_geom(geom_ptr, P, p.coord, nullptr);
 
 	int64_t R = 0;
 	uint32_t max_list = 0;
@@ -244,14 +241,11 @@ static int64_t forward_to_binning(const rgs_camera* cam, const FwdParams& p, int
 		R = (int64_t)box[0];
 		max_list = box[1];
 	}
-	static const bool force_radix = getenv("RGS_BINNING") != nullptr && std::string(getenv("RGS_BINNING")) == "radix";
-	const bool tile_path = !force_radix;  // lists longer than the shared-memory sort take the multi-CTA path inside launch_tile_binning
-	const size_t sort_bytes = (R > 0 && !tile_path) ? sort_temp_bytes((size_t)R) : 0;
 	size_t bin_bytes = 0;
-	carve_bin(nullptr, (size_t)R, tiles, sort_bytes, &bin_bytes);
+	carve_bin(nullptr, (size_t)R, tiles, &bin_bytes);
 	char* bin_ptr = bufs->binning(bufs->binning_user, bin_bytes);
 	if (!bin_ptr) return fail(RGS_E_ALLOC, "binning buffer callback returned NULL");
-	b = carve_bin(bin_ptr, (size_t)R, tiles, sort_bytes, nullptr);
+	b = carve_bin(bin_ptr, (size_t)R, tiles, nullptr);
 	// forward-render writes a ballot word only for the chunks a warp actually tested; backward masks every position at or
 	// behind the warp's last contributor, so the unwritten words never matter -- zero them anyway (<= R bytes) so that no
 	// consumer (debug views, initcheck) ever sees memory the library did not write
@@ -259,14 +253,10 @@ static int64_t forward_to_binning(const rgs_camera* cam, const FwdParams& p, int
 
 	if (P == 0) {
 		RGS_CUDA_TRY(cudaMemsetAsync(img.ranges, 0, (size_t)tiles * sizeof(uint2), s));
-	} else if (tile_path) {
+	} else {
+		// lists longer than the shared-memory sort take the multi-CTA path inside launch_tile_binning
 		StageScope sc(ST_BINNING, s);
 		launch_tile_binning(p, g, b, img, radii, R, max_list, s);
-	} else {
-		// cross-check only (RGS_BINNING=radix): the reference's own scheme, Gaussian-major offsets + one global 45-bit sort
-		StageScope sc(ST_BINNING, s);
-		launch_scan(g, P, s);
-		launch_binning(p, g, b, img, radii, R, s);
 	}
 	if ((rc = debug_sync(cam, s, "binning")) != RGS_OK) return rc;
 	return R;
@@ -358,10 +348,8 @@ static int backward_views(const rgs_camera* cam, const rgs_gaussians* gs, const 
 	if (rc != RGS_OK) return rc;
 	if (!in || !in->geom_buffer || !in->image_buffer) return fail(RGS_E_INVALID, "null backward inputs / buffers");
 	const size_t N = (size_t)p.W * p.Hs;
-	const size_t scan_bytes = p.P > 0 ? scan_temp_bytes(p.P) : 0;
-	g = carve_geom(const_cast<char*>(in->geom_buffer), p.P, p.coord, scan_bytes, nullptr);
-	const size_t sort_bytes = in->num_rendered > 0 ? sort_temp_bytes((size_t)in->num_rendered) : 0;
-	b = carve_bin(const_cast<char*>(in->binning_buffer), (size_t)in->num_rendered, p.grid_x * p.grid_y, sort_bytes, nullptr);
+	g = carve_geom(const_cast<char*>(in->geom_buffer), p.P, p.coord, nullptr);
+	b = carve_bin(const_cast<char*>(in->binning_buffer), (size_t)in->num_rendered, p.grid_x * p.grid_y, nullptr);
 	img = carve_img(const_cast<char*>(in->image_buffer), p.grid_x, p.grid_y, N, p.coord, p.depth, nullptr);
 	return RGS_OK;
 }
@@ -459,7 +447,7 @@ int32_t rgs_backward(const rgs_camera* cam, const rgs_gaussians* gs, const rgs_b
 	// The zero-fill of the dense gradient tensors (pure HBM writes, ~280 MB at 1 M Gaussians) runs on a side stream underneath the
 	// issue-bound backward blend; everything queued on `s` before this call is ordered before it (the tensors may be recycled memory).
 	bool prefilled = false;
-	SideStream* ss = (backward_preprocess_is_compacted() && !cam->debug) ? side_stream() : nullptr;
+	SideStream* ss = !cam->debug ? side_stream() : nullptr;
 	if (ss) {
 		FwdParams p;
 		int rc0 = make_params(cam, gs, p);
@@ -579,16 +567,10 @@ int32_t rgs_debug_get_views(const rgs_camera* cam, int32_t P, int64_t num_render
 	if (!cam || !views) return fail(RGS_E_INVALID, "null pointer");
 	const bool coord = cam->require_coord != 0, depth = cam->require_depth != 0;
 	const int grid_x = (cam->width + TILE_X - 1) / TILE_X, grid_y = (cam->height + TILE_Y - 1) / TILE_Y;
-	size_t N = (size_t)cam->width * cam->height;
-	if (cam->compact_slab) {
-		const int r1 = cam->tile_row_end < 0 ? grid_y : cam->tile_row_end;
-		const int hs = (r1 * TILE_Y < cam->height ? r1 * TILE_Y : cam->height) - cam->tile_row_begin * TILE_Y;
-		N = (size_t)cam->width * (hs > 0 ? hs : 0);
-	}
-	const size_t scan_bytes = P > 0 ? scan_temp_bytes(P) : 0;
-	GeomView g = carve_geom(const_cast<char*>(geom_buffer), P, coord, scan_bytes, nullptr);
-	const size_t sort_bytes = num_rendered > 0 ? sort_temp_bytes((size_t)num_rendered) : 0;
-	BinView b = carve_bin(const_cast<char*>(binning_buffer), (size_t)num_rendered, grid_x * grid_y, sort_bytes, nullptr);
+	const int row_end = cam->tile_row_end < 0 ? grid_y : cam->tile_row_end;
+	const size_t N = (size_t)cam->width * stored_height(cam, cam->tile_row_begin, row_end);
+	GeomView g = carve_geom(const_cast<char*>(geom_buffer), P, coord, nullptr);
+	BinView b = carve_bin(const_cast<char*>(binning_buffer), (size_t)num_rendered, grid_x * grid_y, nullptr);
 	ImgView img = carve_img(const_cast<char*>(image_buffer), grid_x, grid_y, N, coord, depth, nullptr);
 	views->point_list = b.point_list;
 	views->point_list_keys = b.keys_sorted;

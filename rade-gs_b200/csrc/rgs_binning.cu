@@ -1,114 +1,21 @@
-// rgs_binning.cu -- instance expansion, (tile | depth) key sort and per-tile ranges.
+// rgs_binning.cu -- per-tile instance counts and ranges, (tile | depth) key sort, tile-bucket binning.
 //
 // Replaces cub::DeviceScan::InclusiveSum + duplicateWithKeys + cub::DeviceRadixSort::SortPairs +
 // identifyTileRanges (reference: cuda_rasterizer/rasterizer_impl.cu:350, 70-111, 373-381, 151-173).
 //
 // Contract kept bit-exact with the reference: key = (tile_id << 32) | float_bits(view z), value = Gaussian
-// index, instances of one Gaussian are emitted y-major then x, and the sort is stable over the bits
-// [0, 32 + msb(tiles)) -- so equal (tile, depth) pairs stay in ascending Gaussian index.
-#include <cub/cub.cuh>
-
+// index, and the order is the reference's stable sort of instances emitted in ascending Gaussian index -- so
+// equal (tile, depth) pairs stay in ascending Gaussian index.
 #include "rgs_common.cuh"
 
 namespace rgs {
 
-size_t scan_temp_bytes(int P) {
-	size_t bytes = 0;
-	cub::DeviceScan::InclusiveSum(nullptr, bytes, (uint32_t*)nullptr, (uint32_t*)nullptr, P);
-	return bytes;
-}
-
-size_t sort_temp_bytes(size_t R) {
-	size_t bytes = 0;
-	cub::DeviceRadixSort::SortPairs(nullptr, bytes, (uint64_t*)nullptr, (uint64_t*)nullptr, (uint32_t*)nullptr, (uint32_t*)nullptr, (int64_t)R);
-	return bytes;
-}
-
-void launch_scan(GeomView g, int P, cudaStream_t s) {
-	size_t bytes = g.scan_temp_bytes;
-	cub::DeviceScan::InclusiveSum(g.scan_temp, bytes, g.tiles_touched, g.offsets, P, s);
-	count_launch(2);
-}
-
-// One thread per Gaussian writes its run of keys (rasterizer_impl.cu:70-111), clipped to the slab rows.
-__global__ void __launch_bounds__(256) emit_keys_kernel(int P, const float* __restrict__ records, int rec_f, const float* __restrict__ depths,
-                                                         const uint32_t* __restrict__ offsets, const int* __restrict__ radii, int grid_x, int grid_y,
-                                                         int row_begin, int row_end, uint64_t* __restrict__ keys, uint32_t* __restrict__ vals) {
-	const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-	if (idx >= P) return;
-	const int r = radii[idx];
-	if (r <= 0) return;
-	uint32_t off = (idx == 0) ? 0 : offsets[idx - 1];
-	if (offsets[idx] == off) return;  // nothing in this slab
-	const float2 xy = *reinterpret_cast<const float2*>(records + (size_t)idx * rec_f);
-	uint2 rmin, rmax;
-	tile_rect(xy, r, grid_x, grid_y, rmin, rmax);
-	const uint32_t dbits = __float_as_uint(depths[idx]);
-	const int y0 = max((int)rmin.y, row_begin), y1 = min((int)rmax.y, row_end);
-	for (int y = y0; y < y1; y++) {
-		for (int x = rmin.x; x < (int)rmax.x; x++) {
-			uint64_t key = (uint64_t)(y * grid_x + x);
-			key <<= 32;
-			key |= dbits;
-			keys[off] = key;
-			vals[off] = idx;
-			off++;
-		}
-	}
-}
-
-// Boundaries of each tile's run in the sorted key list (rasterizer_impl.cu:151-173).
-__global__ void __launch_bounds__(256) tile_ranges_kernel(int64_t L, const uint64_t* __restrict__ keys, uint2* __restrict__ ranges) {
-	const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-	if (idx >= L) return;
-	const uint32_t cur = (uint32_t)(keys[idx] >> 32);
-	if (idx == 0) {
-		ranges[cur].x = 0;
-	} else {
-		const uint32_t prev = (uint32_t)(keys[idx - 1] >> 32);
-		if (cur != prev) {
-			ranges[prev].y = (uint32_t)idx;
-			ranges[cur].x = (uint32_t)idx;
-		}
-	}
-	if (idx == L - 1) ranges[cur].y = (uint32_t)L;
-}
-
-static uint32_t higher_msb(uint32_t n) {  // rasterizer_impl.cu:35-50
-	uint32_t msb = sizeof(n) * 4;
-	uint32_t step = msb;
-	while (step > 1) {
-		step /= 2;
-		if (n >> msb)
-			msb += step;
-		else
-			msb -= step;
-	}
-	if (n >> msb) msb++;
-	return msb;
-}
-
-void launch_binning(const FwdParams& p, GeomView g, BinView b, ImgView img, const int* radii, int64_t R, cudaStream_t s) {
-	const int tiles = p.grid_x * p.grid_y;
-	cudaMemsetAsync(img.ranges, 0, (size_t)tiles * sizeof(uint2), s);
-	count_launch();
-	if (R <= 0) return;
-	emit_keys_kernel<<<(p.P + 255) / 256, 256, 0, s>>>(p.P, g.records, rec_floats(p.coord), g.depths, g.offsets, radii, p.grid_x, p.grid_y,
-	                                                    p.row_begin, p.row_end, b.keys_unsorted, b.point_list_unsorted);
-	const int bit = (int)higher_msb((uint32_t)tiles);
-	size_t bytes = b.sort_temp_bytes;
-	cub::DeviceRadixSort::SortPairs(b.sort_temp, bytes, b.keys_unsorted, b.keys_sorted, b.point_list_unsorted, b.point_list, R, 0, 32 + bit, s);
-	tile_ranges_kernel<<<(unsigned)((R + 255) / 256), 256, 0, s>>>(R, b.keys_sorted, img.ranges);
-	count_launch(2 + 8);
-}
-
-
 // =====================================================================================================================
-// Tile-bucket binning (default path).
+// Tile-bucket binning.
 //
 // The reference sorts all R instances globally on 45-bit (tile | depth) keys: six 8-bit onesweep passes, each
-// reading and writing 12 B per instance.  The same total order is (tile, depth bits, Gaussian index), so it can be
-// produced with one bucketing step and one local sort instead:
+// reading and writing 12 B per instance.  The same total order is (tile, depth bits, Gaussian index), so it is
+// produced here with one bucketing step and one local sort instead:
 //   1. preprocess marks every splat's tile rectangle with +1 / -1 at its four corners on a (grid_y+1) x (grid_x+1)
 //      difference grid (4 red.global.add per splat, whatever the rectangle's size);
 //   2. tile_scan_kernel: 2D prefix sum of that grid = instances per tile, then the exclusive scan of the T counts ->
@@ -121,7 +28,6 @@ void launch_binning(const FwdParams& p, GeomView g, BinView b, ImgView img, cons
 // stable sort yields (instances are emitted in ascending Gaussian index).  Global traffic: 8 B + 8 B + 4 B (+ 8 B
 // for the exported keys) per instance instead of ~156 B.
 // Lists longer than TILE_SORT_CAP (shared-memory capacity) are split over several CTAs: chunk sort + global merge passes (below).
-// The global radix path above is kept only as a cross-check (`RGS_BINNING=radix`).
 // =====================================================================================================================
 
 __global__ void __launch_bounds__(1024) tile_scan_kernel(int grid_x, int grid_y, int* __restrict__ tile_diff, uint32_t* __restrict__ tile_count,

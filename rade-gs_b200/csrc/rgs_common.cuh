@@ -59,11 +59,10 @@ struct GeomView {
 	float* records;          // [P * rec_floats]
 	float* depths;           // [P]  view-space z (its bit pattern is the low half of the sort key)
 	uint32_t* tiles_touched; // [P]
-	uint32_t* offsets;       // [P]  inclusive scan of tiles_touched
+	uint32_t* bwd_rows;      // [P]  backward preprocess: ids of the rows that received a gradient (in no particular order)
 	uint8_t* clamped;        // [P]  bit c set when colour channel c was clamped at 0
 	float* sigma_inv;        // [P * 12] Sigma^-1 substitute of forward (9 floats, column-major) + flags, reused by backward
-	char* scan_temp;         // CUB temp storage
-	size_t scan_temp_bytes;
+	uint32_t* bwd_row_count; // [1]  length of bwd_rows
 };
 
 struct BinView {
@@ -71,10 +70,7 @@ struct BinView {
 	uint64_t* keys_sorted;         // [R]
 	uint32_t* hitmask;             // [(R/32 + tiles + 1) * 8] per 32-instance chunk: one ballot word per 8x4 pixel block of the tile,
 	                               // written by forward-render (which splats can reach alpha >= 1/255 in the block), read by backward
-	uint32_t* point_list_unsorted; // [R]
-	uint64_t* keys_unsorted;       // [R]
-	char* sort_temp;
-	size_t sort_temp_bytes;
+	uint64_t* keys_unsorted;       // [R]  local keys (depth bits << 32 | Gaussian index) in their tile's segment, before the sort
 };
 
 struct ImgView {
@@ -212,12 +208,7 @@ struct FwdParams {
 void launch_preprocess_forward(const FwdParams& p, GeomView g, int* radii, int* tile_diff, cudaStream_t s);
 void launch_mark_visible(int P, const float* means3D, const float* viewmatrix, uint8_t* present, cudaStream_t s);
 
-size_t scan_temp_bytes(int P);
-size_t sort_temp_bytes(size_t R);
-// inclusive scan of tiles_touched -> offsets; writes the total to *total_dev (pinned or device memory)
-void launch_scan(GeomView g, int P, cudaStream_t s);
-void launch_binning(const FwdParams& p, GeomView g, BinView b, ImgView img, const int* radii, int64_t R, cudaStream_t s);
-// tile-bucket binning (default path): per-tile counts -> ranges/totals -> scatter -> per-tile shared-memory sort
+// tile-bucket binning: per-tile counts -> ranges/totals -> scatter -> per-tile shared-memory sort
 constexpr int TILE_SORT_CAP = 8192;   // longest tile list the one-CTA shared-memory sort takes (2 x 64 KB ping-pong); longer lists: multi-CTA chunk sort + merge
 void launch_tile_scan(const FwdParams& p, ImgView img, cudaStream_t s);
 void launch_tile_binning(const FwdParams& p, GeomView g, BinView b, ImgView img, const int* radii, int64_t R, uint32_t max_list, cudaStream_t s);
@@ -242,7 +233,6 @@ struct ParamGradOut {
 void launch_preprocess_backward(const FwdParams& p, GeomView g, const int* radii, const float* grad_accum, ParamGradOut out, cudaStream_t s,
                                 bool prefilled = false);
 void launch_backward_zero_fill(const FwdParams& p, ParamGradOut out, cudaStream_t s);
-bool backward_preprocess_is_compacted();
 
 // fused activations / densification statistics (rgs_activation.cu; SURVEY.md 8f row 1)
 void launch_activate_forward(int P, const float* raw_scaling, const float* raw_opacity, const float* raw_rotation, const float* filter_3D, float* scales,

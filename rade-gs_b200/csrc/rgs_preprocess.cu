@@ -109,8 +109,8 @@ __device__ __forceinline__ float3 sh_to_rgb(int deg, int M, const float* __restr
 	return float3{fmaxf(res[0], 0.0f), fmaxf(res[1], 0.0f), fmaxf(res[2], 0.0f)};
 }
 
-template <int MIN_BLOCKS>
-__global__ void __launch_bounds__(256, MIN_BLOCKS) preprocess_forward_kernel(FwdParams p, GeomView g, int* __restrict__ radii, int* __restrict__ tile_diff) {
+// 64 registers, 4 CTAs per SM: 5-10 % faster than 3 CTAs per SM on C2 / C3
+__global__ void __launch_bounds__(256, 4) preprocess_forward_kernel(FwdParams p, GeomView g, int* __restrict__ radii, int* __restrict__ tile_diff) {
 	const int idx = blockIdx.x * blockDim.x + threadIdx.x;
 	if (idx >= p.P) return;
 
@@ -281,9 +281,7 @@ __global__ void __launch_bounds__(256, MIN_BLOCKS) preprocess_forward_kernel(Fwd
 void launch_preprocess_forward(const FwdParams& p, GeomView g, int* radii, int* tile_diff, cudaStream_t s) {
 	const int threads = 256;
 	const int blocks = (p.P + threads - 1) / threads;
-	static const int min_blocks = getenv("RGS_PRE_MINBLOCKS") ? atoi(getenv("RGS_PRE_MINBLOCKS")) : 4;  // 64 registers, 4 CTAs/SM: 5-10% faster than 3 (A/B on C2 / C3)
-	if (min_blocks >= 4) preprocess_forward_kernel<4><<<blocks, threads, 0, s>>>(p, g, radii, tile_diff);
-	else preprocess_forward_kernel<3><<<blocks, threads, 0, s>>>(p, g, radii, tile_diff);
+	preprocess_forward_kernel<<<blocks, threads, 0, s>>>(p, g, radii, tile_diff);
 	count_launch();
 }
 

@@ -13,7 +13,7 @@
 //     RGS_FIX_MIP_GRADIENT to use the true opacity*coef instead (off by default: parity first);
 //   * gradients are w.r.t. the quaternion as given (no normalisation inside, backward.cu:554);
 //   * Sigma's eigen-decomposition follows the reference's solver and stopping rules (see rgs_geom.cuh).
-#include <string>
+#include <cstdlib>
 
 #include "rgs_geom.cuh"
 
@@ -322,7 +322,7 @@ __device__ __forceinline__ void preprocess_backward_row(const FwdParams& p, cons
 			dL_dmean.z += d1.z + d2.z;
 		}
 
-		// (the SH term of dL_dmean and dL_dsh are produced by sh_backward_kernel, launched right after this kernel)
+		// (the SH term of dL_dmean and dL_dsh are produced by sh_backward_rows_kernel, launched right after this kernel)
 		o_mean3D[0] = dL_dmean.x; o_mean3D[1] = dL_dmean.y; o_mean3D[2] = dL_dmean.z;
 
 		// ---- covariance -> scale / rotation (backward.cu:492-555) ----
@@ -366,17 +366,9 @@ __device__ __forceinline__ void preprocess_backward_row(const FwdParams& p, cons
 	*reinterpret_cast<float4*>(out.d_rotations + 4 * idx) = make_float4(o_rot[0], o_rot[1], o_rot[2], o_rot[3]);
 }
 
-// dense form: one thread per Gaussian (every output row written, zeros included)
-__global__ void __launch_bounds__(128, 4) preprocess_backward_kernel(FwdParams p, GeomView g, const int* __restrict__ radii,
-                                                                   const float* __restrict__ grad_accum, ParamGradOut out, int fix_mip) {
-	const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-	if (idx >= p.P) return;
-	preprocess_backward_row(p, g, radii, grad_accum, out, fix_mip, idx);
-}
-
-// compacted form: one thread per LISTED Gaussian (rendered and with a non-zero accumulator row); the outputs of all other rows were
-// zero-filled by the launcher.  In a dense scene most rendered splats are occluded in any one view (C2: 84 %, C3: 92 % of the
-// visible ones receive nothing), and a warp of the dense kernel runs the whole chain if ANY of its 32 rows needs it.
+// One thread per LISTED Gaussian (rendered and with a non-zero accumulator row); the outputs of all other rows were zero-filled
+// before.  In a dense scene most rendered splats are occluded in any one view (C2: 84 %, C3: 92 % of the visible ones receive
+// nothing), and a warp of a thread-per-Gaussian kernel would run the whole chain if ANY of its 32 rows needed it.
 __global__ void __launch_bounds__(128, 4) preprocess_backward_rows_kernel(FwdParams p, GeomView g, const int* __restrict__ radii,
                                                                         const float* __restrict__ grad_accum, ParamGradOut out, int fix_mip,
                                                                         const uint32_t* __restrict__ list, const uint32_t* __restrict__ count) {
@@ -422,11 +414,10 @@ __global__ void __launch_bounds__(256) nonzero_rows_kernel(int P, const int* __r
 	if ((keep >> lane) & 1u) list[base + __popc(keep & ((1u << lane) - 1u))] = (uint32_t)idx;
 }
 
-// ---- SH backward (backward.cu:21-140): warp-cooperative so the [M,3] rows move through shared memory coalesced ------
-// A warp owns 32 consecutive Gaussians = one contiguous 32*3M-float block of `shs` and of `dL_dsh`.  The block is
-// copied global -> shared with unit-stride 128-bit loads, each lane then works on its own row (row stride padded to
-// an odd number of floats: conflict-free), overwrites it in place with dL_dsh, and the block streams back coalesced.
-// The view-direction term is added to dL_dmeans3D (third part of the mean gradient, backward.cu:131-139).
+// ---- SH backward (backward.cu:21-140) ----------------------------------------------------------------------------------
+// dL_dsh of every listed Gaussian, and the view-direction term added to dL_dmeans3D (third part of the mean gradient,
+// backward.cu:131-139).  Each lane works on its coefficient row in a shared-memory scratch row (row stride padded to an odd
+// number of floats: conflict-free).
 constexpr int SH_WARPS = 8;
 
 // SH backward of ONE Gaussian whose [M,3] coefficient row sits at `sh` (shared memory): the row is overwritten with dL_dsh and the
@@ -499,85 +490,9 @@ __device__ __forceinline__ void sh_backward_row(float* sh, int idx, int D, int M
 	dm[2] += (-dir_orig.x * dir_orig.z * dL_ddir.x - dir_orig.y * dir_orig.z * dL_ddir.y + (sum2 - dir_orig.z * dir_orig.z) * dL_ddir.z) * invsum32;
 }
 
-
-
-// `count` rows of `width` floats, contiguous in global memory, <-> columns [col0, col0 + width) of the padded shared tile
-// `rows` (loads only): bit r set = row r is wanted; the 16-byte chunks of the other rows are not fetched (their slots are
-// overwritten with zeros by the owner lane afterwards).
-template <bool TO_SHARED>
-__device__ __forceinline__ void sh_block_copy(float* tile, int stride, int col0, int width, int count, const float* src, float* dst, int lane,
-                                              unsigned rows = 0xffffffffu) {
-	const int total = count * width;
-	const uintptr_t addr = TO_SHARED ? reinterpret_cast<uintptr_t>(src) : reinterpret_cast<uintptr_t>(dst);
-	if ((addr & 15) == 0 && (total & 3) == 0) {
-		for (int e = lane * 4; e < total; e += 128) {
-			float vv[4];
-			if (TO_SHARED) {
-				if (!((rows >> (e / width)) & 1u) && !((rows >> ((e + 3) / width)) & 1u)) continue;
-				const float4 v = __ldg(reinterpret_cast<const float4*>(src + e));
-				vv[0] = v.x; vv[1] = v.y; vv[2] = v.z; vv[3] = v.w;
-			}
-#pragma unroll
-			for (int q = 0; q < 4; q++) {
-				const int r = (e + q) / width, c = (e + q) - r * width;
-				if (TO_SHARED) tile[r * stride + col0 + c] = vv[q];
-				else vv[q] = tile[r * stride + col0 + c];
-			}
-			if (!TO_SHARED) *reinterpret_cast<float4*>(dst + e) = make_float4(vv[0], vv[1], vv[2], vv[3]);
-		}
-	} else {
-		for (int e = lane; e < total; e += 32) {
-			const int r = e / width, c = e - r * width;
-			if (TO_SHARED) { if ((rows >> r) & 1u) tile[r * stride + col0 + c] = __ldg(src + e); }
-			else dst[e] = tile[r * stride + col0 + c];
-		}
-	}
-}
-
-__global__ void __launch_bounds__(SH_WARPS * 32) sh_backward_kernel(int P, int D, int M, const float* __restrict__ means3D, const float* __restrict__ cam_pos,
-                                                                     const float* __restrict__ shs, const float* __restrict__ shs_rest,
-                                                                     const int* __restrict__ radii, const uint8_t* __restrict__ clamped,
-                                                                     const float* __restrict__ grad_accum, int GF, float* __restrict__ d_sh,
-                                                                     float* __restrict__ d_sh_rest, float* __restrict__ d_means3D) {
-	extern __shared__ float s_sh[];
-	const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-	const int row = 3 * M, stride = row | 1;
-	float* tile = s_sh + (size_t)warp * 32 * stride;
-	const int g0 = (blockIdx.x * SH_WARPS + warp) * 32;
-	if (g0 >= P) return;
-	const int count = min(32, P - g0);
-	// split layout (ABI 2): coefficient 0 comes from / goes to the [P,1,3] tensors, bands 1.. the [P,M-1,3] ones
-	const bool split = shs_rest != nullptr;
-	const int w0 = split ? 3 : row;
-	const int idx = g0 + lane;
-	// rows that need their coefficients: rendered AND a non-zero colour gradient after the clamp mask; for all others dL_dsh = 0 and
-	// the view-direction term vanishes, so their 12*M bytes are not read (occluded splats: a large share of a dense scene)
-	bool need = false;
-	if (lane < count && radii[idx] > 0) {
-		const uint8_t cb0 = clamped[idx];
-		const float* ga0 = grad_accum + (size_t)idx * GF + G_COL;
-		need = (!(cb0 & 1) && ga0[0] != 0.f) || (!(cb0 & 2) && ga0[1] != 0.f) || (!(cb0 & 4) && ga0[2] != 0.f);
-	}
-	const unsigned need_mask = __ballot_sync(0xffffffffu, need);
-	sh_block_copy<true>(tile, stride, 0, w0, count, shs + (size_t)g0 * w0, nullptr, lane, need_mask);
-	if (split) sh_block_copy<true>(tile, stride, 3, row - 3, count, shs_rest + (size_t)g0 * (row - 3), nullptr, lane, need_mask);
-	__syncwarp();
-	if (lane < count) {
-		float* sh = tile + lane * stride;
-		if (!need) {
-			for (int i = 0; i < row; i++) sh[i] = 0.f;
-		} else {
-			sh_backward_row(sh, idx, D, M, means3D, cam_pos, clamped, grad_accum, GF, d_means3D);
-		}
-	}
-	__syncwarp();
-	sh_block_copy<false>(tile, stride, 0, w0, count, nullptr, d_sh + (size_t)g0 * w0, lane);
-	if (split) sh_block_copy<false>(tile, stride, 3, row - 3, count, nullptr, d_sh_rest + (size_t)g0 * (row - 3), lane);
-}
-
-// compacted form of the SH backward: lane = one LISTED Gaussian.  The rows are scattered in memory anyway, so every lane fetches its own
-// coefficient row (12*M contiguous bytes: twelve independent 128-bit loads in flight when the layout allows) into its shared-memory
-// scratch row, works on it in place as above and stores dL_dsh back the same way; all other rows of dL_dsh were zero-filled.
+// Lane = one LISTED Gaussian.  The rows are scattered in memory, so every lane fetches its own coefficient row (12*M contiguous bytes:
+// twelve independent 128-bit loads in flight when the layout allows) into its shared-memory scratch row, works on it in place and
+// stores dL_dsh back the same way; all other rows of dL_dsh were zero-filled.
 __global__ void __launch_bounds__(SH_WARPS * 32) sh_backward_rows_kernel(int D, int M, const float* __restrict__ means3D, const float* __restrict__ cam_pos,
                                                                           const float* __restrict__ shs, const float* __restrict__ shs_rest,
                                                                           const uint8_t* __restrict__ clamped, const float* __restrict__ grad_accum, int GF,
@@ -633,12 +548,7 @@ __global__ void __launch_bounds__(SH_WARPS * 32) sh_backward_rows_kernel(int D, 
 	}
 }
 
-bool backward_preprocess_is_compacted() {
-	static const bool dense = getenv("RGS_BWD_PREPROCESS") != nullptr && std::string(getenv("RGS_BWD_PREPROCESS")) == "dense";
-	return !dense;
-}
-
-// zero-fill of the nine dense gradient tensors (what the compacted kernels do not write).  Pure HBM writes: rgs_backward issues it on
+// zero-fill of the nine dense gradient tensors (what the row kernels do not write).  Pure HBM writes: rgs_backward issues it on
 // a side stream so that it runs underneath the issue-bound backward blend.
 void launch_backward_zero_fill(const FwdParams& p, ParamGradOut out, cudaStream_t s) {
 	const size_t P = (size_t)p.P;
@@ -660,31 +570,11 @@ void launch_backward_zero_fill(const FwdParams& p, ParamGradOut out, cudaStream_
 void launch_preprocess_backward(const FwdParams& p, GeomView g, const int* radii, const float* grad_accum, ParamGradOut out, cudaStream_t s,
                                 bool prefilled) {
 	static const int fix_mip = getenv("RGS_FIX_MIP_GRADIENT") != nullptr && atoi(getenv("RGS_FIX_MIP_GRADIENT")) != 0;
-	const bool dense = !backward_preprocess_is_compacted();
 	const bool has_sh = p.shs != nullptr && out.d_sh != nullptr && p.M > 0;
-	const int stride = (3 * p.M) | 1;
-	const size_t smem = (size_t)SH_WARPS * 32 * stride * sizeof(float);
-	static size_t configured[64] = {}, configured_rows[64] = {};
-	if (dense || g.scan_temp == nullptr || g.scan_temp_bytes < sizeof(uint32_t)) {
-		// every row through the full chain (kept as a cross-check: RGS_BWD_PREPROCESS=dense)
-		preprocess_backward_kernel<<<(p.P + 127) / 128, 128, 0, s>>>(p, g, radii, grad_accum, out, fix_mip);
-		count_launch();
-		if (has_sh) {
-			if (smem > 48 * 1024) ensure_dynamic_smem(sh_backward_kernel, smem, configured);
-			const int per_block = SH_WARPS * 32;
-			sh_backward_kernel<<<(p.P + per_block - 1) / per_block, per_block, smem, s>>>(p.P, p.D, p.M, p.means3D, p.cam_pos, p.shs, p.shs_rest, radii,
-			                                                                               g.clamped, grad_accum, grad_floats(p.coord), out.d_sh,
-			                                                                               out.d_sh_rest, out.d_means3D);
-			count_launch();
-		}
-		return;
-	}
-	// compacted: zero-fill the outputs (memsets run at HBM write speed), list the rows that received anything, run the chains on those.
-	// The list lives in the geometry buffer's `offsets` array (only the cross-check radix path of forward uses it), its length in the
-	// first word of the scan scratch.
+	// zero-fill the outputs (memsets run at HBM write speed), list the rows that received anything, run the chains on those
 	if (!prefilled) launch_backward_zero_fill(p, out, s);
-	uint32_t* list = g.offsets;
-	uint32_t* count = reinterpret_cast<uint32_t*>(g.scan_temp);
+	uint32_t* list = g.bwd_rows;
+	uint32_t* count = g.bwd_row_count;
 	cudaMemsetAsync(count, 0, sizeof(uint32_t), s);
 	const int GF = grad_floats(p.coord);
 	if (GF == GRAD_FLOATS_BASE)
@@ -697,7 +587,9 @@ void launch_preprocess_backward(const FwdParams& p, GeomView g, const int* radii
 	preprocess_backward_rows_kernel<<<rows_grid, 128, 0, s>>>(p, g, radii, grad_accum, out, fix_mip, list, count);
 	count_launch(2 + 8 + (has_sh ? 1 : 0));
 	if (has_sh) {
-		if (smem > 48 * 1024) ensure_dynamic_smem(sh_backward_rows_kernel, smem, configured_rows);
+		const size_t smem = (size_t)SH_WARPS * 32 * ((3 * p.M) | 1) * sizeof(float);
+		static size_t configured[64] = {};
+		if (smem > 48 * 1024) ensure_dynamic_smem(sh_backward_rows_kernel, smem, configured);
 		const int sh_grid = min((p.P + SH_WARPS * 32 - 1) / (SH_WARPS * 32), sms * 8);
 		sh_backward_rows_kernel<<<sh_grid, SH_WARPS * 32, smem, s>>>(p.D, p.M, p.means3D, p.cam_pos, p.shs, p.shs_rest, g.clamped, grad_accum, GF, out.d_sh,
 		                                                            out.d_sh_rest, out.d_means3D, list, count);

@@ -276,7 +276,7 @@ def _oracle_inputs(sc, coord, depth, ks, deg, shs=None):
 def test_long_tile_lists_take_the_multi_cta_sort(n_splats):
     """Tile lists longer than the one-CTA shared-memory sort (8192) are split over several CTAs (chunk sort + global merge
     passes; 2, 3 and 5 passes here, so both ping-pong parities) and must still give the reference order: splats piled onto a
-    few pixels.  No library sort is involved (the global radix path only runs when RGS_BINNING=radix asks for it)."""
+    few pixels.  No library sort is involved: binning is the project's own kernels only."""
     import oracle
     from rade_gs_b200 import rawapi, scenes
     sc = scenes.make_scene(n_splats, 64, 48, 200.0, -4.0, seed=31)

@@ -5,7 +5,6 @@ timeout 600 python tools/stress_determinism.py 120 1 0 0.0 > gpurun_out/f_stress
 timeout 600 python tools/stress_determinism.py 60 1 1 0.1 > gpurun_out/f_stress_both.log 2>&1; tail -2 gpurun_out/f_stress_both.log
 timeout 2400 python -m pytest tests -m gpu -q > gpurun_out/f_pytest.log 2>&1; echo "pytest rc=$?"; grep -E "passed|failed|FAILED|ERROR" gpurun_out/f_pytest.log | tail -12
 timeout 600 python bench.py --steps 20 --warmup 5 > gpurun_out/f_bench_ours.json 2> gpurun_out/f_bench_ours.err; echo "bench ours rc=$?"; tail -3 gpurun_out/f_bench_ours.err
-RGS_BWD_PREPROCESS=dense timeout 600 python bench.py --steps 20 --warmup 5 --no-cpu-baseline > gpurun_out/f_bench_ours_densebwd.json 2> gpurun_out/f_bench_ours_densebwd.err
 for cfg in C3 C4; do timeout 600 python bench.py --steps 10 --warmup 3 --config $cfg --no-cpu-baseline > gpurun_out/f_bench_ours_$cfg.json 2> gpurun_out/f_bench_ours_$cfg.err; echo "bench $cfg rc=$?"; done
 python - <<'PY'
 import json, glob
